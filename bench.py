@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- rendered frames/sec at 64^2 neural x 96 samples -> 512^2 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     (N > 1: python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...)
 
 A "step" is one pass of the hot path over one batch: G.synthesis(ws, c) for 8 latents of the random-init
@@ -18,6 +18,9 @@ roofline : the fused ray-march kernel (dominant kernel of the renderer), timed l
 cpu_baseline : the oracle port (stock torch-CPU ops chained like the reference's free functions) on the host cores,
         bounded sample = 1 frame of the same workload.
 --impl reference : that CPU path as the timed arm (rank 0 only).
+--dump-outputs DIR : after the timed steps, rank 0 writes the images its last timed step returned to DIR/image.npy (float32
+        [8, 3, 512, 512], 25 MB).  Inputs and the ray jitter seed of that step are fixed, so two builds can be compared output
+        for output.
 """
 
 import argparse
@@ -32,6 +35,7 @@ import time
 import numpy as np
 import torch
 
+sys.dont_write_bytecode = True           # the source tree may be read-only: no __pycache__ next to the sources
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
@@ -245,6 +249,7 @@ def main():
     ap.add_argument('--impl', default='ours', choices=['ours', 'reference'])
     ap.add_argument('--cpu-reps', type=int, default=2, help='timed repetitions of the 1-frame CPU baseline')
     ap.add_argument('--no-cpu-baseline', action='store_true')
+    ap.add_argument('--dump-outputs', metavar='DIR', help='write the images of the last timed step to DIR/image.npy')
     args = ap.parse_args()
 
     if args.impl == 'reference':
@@ -300,10 +305,12 @@ def main():
         with ClockSampler(device.index or 0) as clocks:
             barrier()
             torch.cuda.profiler.start()           # no-op unless run under `ncu --profile-from-start off`
-            for a, b in ev:
+            for i, (a, b) in enumerate(ev):
+                if i == len(ev) - 1:
+                    torch.manual_seed(0)          # the step's ray jitter seed is drawn from torch's generator: fix it for --dump-outputs
                 flush.zero_()
                 a.record()
-                step()
+                out = step()
                 b.record()
             barrier()
             torch.cuda.profiler.stop()
@@ -343,6 +350,10 @@ def main():
     if world > 1:
         tdist.all_reduce(t, op=tdist.ReduceOp.MAX)
     dev_ms, e2e_ms = float(t[0]), float(t[1])
+
+    if rank == 0 and args.dump_outputs:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, 'image.npy'), out.float().cpu().numpy())
 
     if rank == 0:
         peak, peak_src = measured_peak_gbs()

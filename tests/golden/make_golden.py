@@ -448,11 +448,68 @@ def g_networks():
     save('networks', **out)
 
 
+# ------------------------------------------------------------------ gen_videos.py frame loop (config 3)
+def g_video_loop():
+    """The (w, camera) pair the reference's gen_interp_video hands to G.synthesis for every (frame, grid cell), recorded from the
+    unmodified frame loop (gen_videos.py:112-129) with seeds [3, 1, 4, 1, 5, 9, 2, 6], w_frames=3, a 2x1 grid, psi 0.7, cutoff 4;
+    the keyframe mapping call (its z, c and the ws it returned, from a small random-init generator); and layout_grid
+    (gen_videos.py:24-38) applied to seeded uint8 frames."""
+    import types
+    from oracle.backend import cpu_reference_ops
+    from ide3d_b200.training.triplane import TriPlaneGenerator
+    for name in ('imageio', 'mrcfile'):                  # output writers the recorded path never reaches
+        sys.modules.setdefault(name, types.ModuleType(name))
+    gv = __import__('gen_videos')
+    torch.manual_seed(0)
+    G = TriPlaneGenerator(z_dim=32, w_dim=32, img_resolution=64, plane_resolution=32, render_size=16, channel_base=512,
+                          channel_max=16, sr_channels=(8, 8), mapping_kwargs=dict(num_layers=2)).eval().requires_grad_(False)
+    calls, mapped = [], {}
+
+    def record_mapping(z, c, **kw):
+        assert kw == dict(truncation_psi=0.7, truncation_cutoff=4)
+        mapped.update(map_z=z, map_c=c, map_ws=G.mapping(z, c, **kw))
+        return mapped['map_ws']
+
+    class Recorder:
+        z_dim = G.z_dim
+
+        def parameters(self):
+            return G.parameters()
+
+        @staticmethod
+        def mapping(z, c, **kw):
+            return record_mapping(z, c, **kw)
+
+        @staticmethod
+        def synthesis(ws, c, **kw):
+            calls.append((ws.detach().clone(), c.detach().clone()))
+            n = ws.shape[0]
+            return torch.zeros(n, 3, 4, 4), torch.zeros(n, 19, 4, 4)
+
+    class Writer:
+        def append_data(self, a):
+            pass
+
+        def close(self):
+            pass
+
+    sys.modules['imageio'].get_writer = lambda *a, **k: Writer()
+    with torch.no_grad(), cpu_reference_ops():
+        gv.gen_interp_video(Recorder(), 'unused.mp4', image_mode='image_seg', device=torch.device('cpu'), seeds=[3, 1, 4, 1, 5, 9, 2, 6],
+                            w_frames=3, grid_dims=(2, 1), psi=0.7, truncation_cutoff=4)
+    calls = calls[1:]                                    # the warm-up call (:89)
+    F, gh, gw = 12, 1, 2
+    assert len(calls) == F * gh * gw
+    frames = torch.randint(0, 255, (F * gh * gw, 3, 5, 7), dtype=torch.uint8, generator=torch.Generator().manual_seed(0))
+    grids = np.stack([gv.layout_grid(frames[f * gh * gw:(f + 1) * gh * gw], grid_w=gw, grid_h=gh, float_to_uint8=False) for f in range(F)])
+    save('video_loop', ws=torch.cat([w for w, _ in calls]), c=torch.cat([c for _, c in calls]), frames=frames, grids=grids, **mapped)
+
+
 if __name__ == '__main__':
     torch.set_num_threads(4)
     fns = dict(rays=g_rays, transform=g_transform, camera=g_camera, triplane=g_triplane, integration=g_integration, pdf=g_pdf,
                chain=g_chain, chain_hier=g_chain_hier, create_samples=g_create_samples, bias_act=g_bias_act, upfirdn2d=g_upfirdn2d,
-               filtered_lrelu=g_filtered_lrelu, conv2d_resample=g_conv2d_resample, networks=g_networks)
+               filtered_lrelu=g_filtered_lrelu, conv2d_resample=g_conv2d_resample, networks=g_networks, video_loop=g_video_loop)
     for name in (sys.argv[1:] or list(fns)):              # `make_golden.py networks` regenerates one fixture only
         fns[name]()
     print('all reference outputs reproduced by oracle/ within tolerance')

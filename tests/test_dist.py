@@ -57,16 +57,25 @@ def test_shard_helpers():
 
 
 @pytest.mark.timeout(300)
-def test_two_rank_gloo_frame_and_slab_gather():
+def test_two_rank_gloo_frame_and_slab_gather(monkeypatch):
+    # the ranks stay on the CPU on a GPU machine too: init_from_env would bind rank r to cuda:r, which a one-GPU machine lacks
+    monkeypatch.setenv('CUDA_VISIBLE_DEVICES', '')
     ctx = mp.get_context('spawn')
     q = ctx.Queue()
     port = 29500 + (os.getpid() % 2000)
     procs = [ctx.Process(target=_worker, args=(r, 2, port, q)) for r in range(2)]
     for p in procs:
         p.start()
-    res = [q.get(timeout=240) for _ in procs]
+    try:
+        res = [q.get(timeout=240) for _ in procs]
+        for p in procs:
+            p.join(timeout=60)
+    finally:
+        for p in procs:                                  # a rank whose peer died waits in the rendezvous: do not leave it behind
+            if p.is_alive():
+                p.kill()
+                p.join()
     for p in procs:
-        p.join(timeout=60)
         assert p.exitcode == 0
     for rank, shape, diff, same_vol in res:
         assert tuple(shape) == (5, 3, 32, 32) and diff <= 1 and same_vol, (rank, shape, diff, same_vol)

@@ -1,12 +1,10 @@
 """North-star target (BASELINE.json): the fused ray-march >= 20x the reference renderer's single-GPU frames/s at
 64^2 x 96 samples.  The "reference renderer on the GPU" is the reference's own op chain -- a1 rays, a2 jitter,
 a3 cam2world bmm, a5 F.grid_sample x 6, decoder matmuls, a7 compositing -- executed by the oracle on CUDA tensors
-(every stage materialised in HBM, as volumetric_rendering.py does).  The measured ratio is written to
-gpurun_out/renderer_speedup.json.  Round-1 status: 11.0x measured on B200 (composed chain 16.6 ms, fused 1.51 ms per
-8 frames) -- the 20x target is NOT met yet; the assertion below only guards the measured level against regressions."""
+(every stage materialised in HBM, as volumetric_rendering.py does).  The measured ratio is printed (pytest -s).
+Round-1 status: 11.0x measured on B200 (composed chain 16.6 ms, fused 1.51 ms per 8 frames) -- the 20x target is NOT met yet; the assertion below only guards the measured level against regressions."""
 
 import json
-import os
 
 import pytest
 import torch
@@ -63,10 +61,7 @@ def test_fused_renderer_vs_composed_reference_chain_on_gpu():
     ratio = ms_ref / ms_fused
     rec = dict(frames=N, num_steps=S, composed_reference_chain_ms=ms_ref, fused_ms=ms_fused, speedup=ratio,
                composed_fps=N / ms_ref * 1e3, fused_fps=N / ms_fused * 1e3, max_abs_feature_diff=err)
-    os.makedirs('gpurun_out', exist_ok=True)
-    with open('gpurun_out/renderer_speedup.json', 'w') as f:
-        json.dump(rec, f, indent=1)
-    print(rec)
+    print(json.dumps(rec))
     assert err < 3e-4
     assert (depth.reshape(N, -1) - depth_ref.reshape(N, -1)).abs().max().item() < 1e-4
     assert ratio >= 8.0, rec          # north-star target is 20; see the module docstring
